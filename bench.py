@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- denoise-steps/sec of the FRESCO hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl fresco|reference] [--workload ...]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl fresco|reference] [--workload ...] [--dump-outputs DIR]
 
 A "step" is one UNet forward of an SD-1.5-shaped random-init fp16 UNet with the FRESCO hooks installed through the
 reference's own plug-in surface (apply_FRESCO_attn / apply_FRESCO_opt -> pipe.unet(...)):
@@ -348,6 +348,7 @@ def dist_setup():
 
 
 def timed_region(wl, steps, warmup, host_io, world):
+    """(ms of the `steps` timed steps, the output of the last one)"""
     import torch.distributed as dist
     for k in range(warmup):
         wl.step(k, host_io)
@@ -358,8 +359,9 @@ def timed_region(wl, steps, warmup, host_io, world):
     e0 = torch.cuda.Event(enable_timing=True)
     e1 = torch.cuda.Event(enable_timing=True)
     e0.record()
+    out = None
     for k in range(steps):
-        wl.step(k, host_io)
+        out = wl.step(k, host_io)
     e1.record()
     torch.cuda.synchronize()
     if world > 1:
@@ -369,7 +371,16 @@ def timed_region(wl, steps, warmup, host_io, world):
         t = torch.tensor([ms], device="cuda")
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t.item())
-    return ms
+    return ms, out
+
+
+def dump_outputs(directory, arrays):
+    """--dump-outputs: every array as <directory>/<name>.npy in float32, so that two builds can be compared output for
+    output on the same seeded inputs"""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), t.detach().float().cpu().numpy())
 
 
 # --------------------------------------------------------------------------------------------
@@ -540,7 +551,11 @@ def main():
                     help="replay the step from CUDA graphs (auto: on for the frame-sharded workload)")
     ap.add_argument("--profile-mode", action="store_true",
                     help="for ncu captures only: 1 warm-up + --steps, no e2e / cpu baseline; never a bench value")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last timed step's output to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "fresco" and not args.profile_mode:
         args.warmup = max(args.warmup, 3)
 
@@ -634,11 +649,15 @@ def main():
     ops.PROFILE = [] if wl.graphs is None else None
     launches0 = _lib.launch_count()
     sampler.start()
-    ms = timed_region(wl, args.steps, args.warmup, False, world)
+    ms, last_out = timed_region(wl, args.steps, args.warmup, False, world)
     clocks = sampler.stop()
     launches = _lib.launch_count() - launches0
     prof = ops.PROFILE
     ops.PROFILE = None
+    if args.dump_outputs:
+        # the noise prediction of the last timed step (a rank's frame shard when sharded); saved before any further step
+        # can overwrite a graph's static output buffer
+        dump_outputs(args.dump_outputs, {"noise_pred" if world == 1 else "noise_pred_rank%d" % rank: last_out})
     prof_steps = args.steps + args.warmup
     if wl.graphs is not None:
         # launches inside a replayed graph are not seen by the library's counter: count one eager cycle instead, and
@@ -661,7 +680,7 @@ def main():
         print(json.dumps({"profile_mode": True, "ms_per_step": ms / args.steps, "note": "not a bench value"}))
         return
     # ---- e2e: pinned-host inputs / outputs copied inside the timed region
-    ms_e2e = timed_region(wl, args.steps, 1, True, world)
+    ms_e2e, _ = timed_region(wl, args.steps, 1, True, world)
 
     units = (n_frames / float(N_FRAMES)) if workload in ("config4", "config4opt", "config5") else (world if replicas else 1)
     value = units * args.steps / (ms / 1000.0)

@@ -1,8 +1,8 @@
-"""Generate golden vectors by running the REAL reference (/root/reference) on CPU.
+"""Generate golden vectors by running the REAL reference (the original FRESCO project) on CPU.
 
-Run in the build container only (the reference is not present on the GPU box):
+Only regenerating the fixtures needs the original project; the tests read the committed .npz files:
 
-    python tests/golden/make_golden.py
+    FRESCO_REFERENCE_DIR=<checkout of FRESCO> python tests/golden/make_golden.py [--set b | --set control]
 
 The reference imports two diffusers names and matplotlib at module top
 (src/diffusion_hacked.py:7-8, src/utils.py:5); neither is used on the path we
@@ -19,7 +19,7 @@ import torch
 import torch.nn.functional as F
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REF = "/root/reference"
+REF = os.environ.get("FRESCO_REFERENCE_DIR", "")
 
 
 def import_reference():
@@ -36,6 +36,8 @@ def import_reference():
             for k, v in attrs.items():
                 setattr(m, k, v)
             sys.modules[name] = m
+    if not os.path.isdir(REF):
+        raise SystemExit("set FRESCO_REFERENCE_DIR to a checkout of the original FRESCO project")
     os.chdir(REF)
     sys.path.insert(0, REF)
     import src.diffusion_hacked as dh   # noqa
@@ -158,10 +160,50 @@ def scenario_b(dh, fu, geometry, matching, ut):
     print("golden fixture set B written to", HERE)
 
 
+def control_sequence():
+    """The operations AttentionControl is driven through: store, replay of the stored features with wrap-around of the
+    ring index, every enable / disable, re-enabling with and without new parameters, clear_store."""
+    t = [torch.full((1,), float(i)) for i in range(6)]
+    return [("enable_controller", ()), ("enable_store", ()), ("call", (t[0],)), ("call", (t[1],)), ("call", (t[2],)),
+            ("disable_store", ()), ("enable_intraattn", ()), ("call", (None,)), ("call", (None,)), ("call", (None,)),
+            ("call", (None,)), ("enable_cfattn", ([torch.ones(2, 4, dtype=torch.bool)],)),
+            ("enable_interattn", ({"fwd_mappings": [1]},)), ("disable_interattn", ()), ("enable_interattn", ()),
+            ("disable_controller", ()), ("enable_controller", ()), ("clear_store", ()), ("enable_intraattn", ()),
+            ("call", (t[3],))]
+
+
+def control_trace(ctrl):
+    """control_sequence() applied to `ctrl`: the operation names; after every operation (store, index, use_intraattn,
+    use_interattn, use_cfattn, number of stored features); what each call returned (NaN for None); and the bias / scale
+    attributes at the end."""
+    ops, states, returned = [], [], []
+    for name, args in control_sequence():
+        if name == "call":
+            r = ctrl(*args)
+            returned.append(float("nan") if r is None else r.item())
+        else:
+            getattr(ctrl, name)(*args)
+        ops.append(name)
+        states.append((ctrl.store, ctrl.index, ctrl.use_intraattn, ctrl.use_interattn, ctrl.use_cfattn,
+                       len(ctrl.stored_attn["decoder_attn"])))
+    attrs = (ctrl.intraattn_bias, ctrl.intraattn_scale_factor, ctrl.interattn_scale_factor)
+    return {"ops": np.array(ops), "states": np.array(states, dtype=np.int64),
+            "returned": np.array(returned, dtype=np.float64), "attrs": np.array(attrs, dtype=np.float64)}
+
+
+def scenario_control(dh):
+    """The reference's AttentionControl (src/diffusion_hacked.py:23-137) through control_sequence()."""
+    np.savez_compressed(os.path.join(HERE, "attention_control.npz"), **control_trace(dh.AttentionControl()))
+    print("golden AttentionControl trace written to", HERE)
+
+
 def main():
     dh, fu, geometry, matching, ut = import_reference()
-    if "--set" in sys.argv and sys.argv[sys.argv.index("--set") + 1] == "b":
+    which = sys.argv[sys.argv.index("--set") + 1] if "--set" in sys.argv else "a"
+    if which == "b":
         return scenario_b(dh, fu, geometry, matching, ut)
+    if which == "control":
+        return scenario_control(dh)
     torch.manual_seed(0)
     torch.set_grad_enabled(False)
 

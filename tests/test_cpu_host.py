@@ -2,16 +2,16 @@
 the host-side mirror of the reference's hook surface behaves like the reference, and the
 product path refuses to run without CUDA (no silent fallback)."""
 import ctypes
+import importlib.util
 import os
 import re
 import sys
-import types
 
+import numpy as np
 import pytest
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
 
 
 @pytest.fixture(scope="module")
@@ -87,53 +87,19 @@ def test_product_never_imports_oracle():
                 assert "import oracle" not in src and "from oracle" not in src, os.path.join(dp, f)
 
 
-def _import_reference():
-    for name, attrs in (("diffusers", {}), ("diffusers.models", {}),
-                        ("diffusers.models.unet_2d_condition", {"UNet2DConditionOutput": object}),
-                        ("diffusers.models.attention_processor", {"AttnProcessor2_0": object}),
-                        ("matplotlib", {}), ("matplotlib.pyplot", {})):
-        if name not in sys.modules:
-            m = types.ModuleType(name)
-            for k, v in attrs.items():
-                setattr(m, k, v)
-            sys.modules[name] = m
-    cwd = os.getcwd()
-    os.chdir(REF)
-    sys.path.insert(0, REF)
-    try:
-        import src.diffusion_hacked as dh
-    finally:
-        os.chdir(cwd)
-    return dh
-
-
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present")
-def test_attention_control_state_machine_matches_reference():
-    """drive the reference's AttentionControl and ours through the same call sequence"""
-    ref_dh = _import_reference()
+def test_attention_control_state_machine_matches_reference(golden):
+    """drive our AttentionControl through the call sequence the reference's was driven through to make the fixture
+    (tests/golden/make_golden.py --set control) and compare the state after every operation"""
+    spec = importlib.util.spec_from_file_location("make_golden", os.path.join(ROOT, "tests", "golden", "make_golden.py"))
+    make_golden = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(make_golden)
     from fresco_b200 import diffusion_hacked as my_dh
-    a, b = ref_dh.AttentionControl(), my_dh.AttentionControl()
-
-    def snap(c):
-        return (c.store, c.index, c.use_intraattn, c.use_interattn, c.use_cfattn, len(c.stored_attn["decoder_attn"]))
-
-    t = [torch.full((1,), float(i)) for i in range(6)]
-    seq = [("enable_controller", ()), ("enable_store", ()), ("call", (t[0],)), ("call", (t[1],)), ("call", (t[2],)),
-           ("disable_store", ()), ("enable_intraattn", ()), ("call", (None,)), ("call", (None,)), ("call", (None,)),
-           ("call", (None,)), ("enable_cfattn", ([torch.ones(2, 4, dtype=torch.bool)],)),
-           ("enable_interattn", ({"fwd_mappings": [1]},)), ("disable_interattn", ()), ("enable_interattn", ()),
-           ("disable_controller", ()), ("enable_controller", ()), ("clear_store", ()), ("enable_intraattn", ()),
-           ("call", (t[3],))]
-    for name, args in seq:
-        if name == "call":
-            ra, rb = a(*args), b(*args)
-            assert (ra is None and rb is None) or torch.equal(ra, rb)
-        else:
-            getattr(a, name)(*args)
-            getattr(b, name)(*args)
-        assert snap(a) == snap(b), (name, snap(a), snap(b))
-    for attr in ("intraattn_bias", "intraattn_scale_factor", "interattn_scale_factor"):
-        assert getattr(a, attr) == getattr(b, attr)
+    want, got = golden("attention_control"), make_golden.control_trace(my_dh.AttentionControl())
+    assert want["ops"].tolist() == got["ops"].tolist()
+    for i, name in enumerate(got["ops"]):
+        assert want["states"][i].tolist() == got["states"][i].tolist(), (i, name, want["states"][i], got["states"][i])
+    assert np.array_equal(want["returned"], got["returned"], equal_nan=True), (want["returned"], got["returned"])
+    assert want["attrs"].tolist() == got["attrs"].tolist()
 
 
 def test_hook_surface_on_harness_unet():
